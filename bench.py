@@ -193,6 +193,29 @@ def time_solver(solver, steps, warmup, flush, barrier, torch):
     return ts, last, solver.batch.launch_count() - l0, per
 
 
+DUMP_LIMIT = 64 * 1024 * 1024
+DUMP_SEQ_AXIS = {"samples": 0, "frames": 0, "success": 0, "stage_status": 1, "stage_iters": 1}
+
+
+def dump_outputs(out, path):
+    """Writes the arrays `ShardedSolver.solve` returned (sampled trajectories, per-sequence status) as <path>/<name>.npy in
+    float64, in the caller's layout, so that two builds can be compared output for output.  Above DUMP_LIMIT bytes every
+    array keeps the same fixed, seeded sample of sequences, whose indices go to sequence_index.npy.
+    Compare with tolerances: the kernels accumulate with fp64 atomics, so two runs of one build already differ.  On a B200,
+    64 x 120-frame sequences, two runs differed by ~1e-9 m / 1e-6 N per sequence, and by 2e-4 m / 2e-2 N in the one
+    sequence whose stage-3 iteration count changed (the tolerances of tests/test_phys_gpu.py allow 5e-3 m / 5 N)."""
+    arrays = {k: np.asarray(out[k], dtype=np.float64) for k in DUMP_SEQ_AXIS}
+    n = arrays["frames"].shape[0]
+    keep = int(DUMP_LIMIT // (sum(a.nbytes for a in arrays.values()) / n + 8))
+    if keep < n:
+        idx = np.sort(np.random.default_rng(0).choice(n, keep, replace=False))
+        arrays = {k: np.take(a, idx, axis=DUMP_SEQ_AXIS[k]) for k, a in arrays.items()}
+        arrays["sequence_index"] = idx.astype(np.float64)
+    os.makedirs(path, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(path, k + ".npy"), a)
+
+
 def run_contact(args):
     """BASELINE.json configs[2] (contact-net inference, 100k windows, 1 B200): scripts/bench_contact.py emits the line."""
     cmd = [sys.executable, os.path.join(ROOT, "scripts", "bench_contact.py"), "--steps", str(args.steps), "--warmup", str(args.warmup)]
@@ -213,7 +236,13 @@ def main():
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-named", action="store_true", help="skip the 1024-sequence pass at 8 GPUs")
     ap.add_argument("--named-world", type=int, default=8, help="world size at which the 128-per-GPU pass runs (8 = BASELINE configs[3])")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one returned as DIR/<name>.npy (float64, at most 64 MiB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.workload == "contact" or args.impl == "reference"):
+        ap.error("--dump-outputs writes the product arm's phys-optim results (--workload phys or long)")
     rank, world, local = _env_int("RANK", 0), _env_int("WORLD_SIZE", 1), _env_int("LOCAL_RANK", 0)
     if args.workload == "contact":
         if rank == 0:
@@ -413,6 +442,8 @@ def main():
                                     "sample": "%d sequences x %d frames (seeds 0..%d of the workload's generator), one per core on %d cores, "
                                               "full staged solve, %.1f s wall" % (len(seeds), fr_, len(seeds) - 1, cores, wall),
                                     "residual": rc}
+        if args.dump_outputs:
+            dump_outputs(last, args.dump_outputs)
         print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()

@@ -5,8 +5,10 @@ only.  Writes tests/golden/kinopt/:
   inputs.npz      synthetic clip: 2D keypoints + confidences, root-relative 3D joints, root translation, initial joint
                   angles (axis-angle, SMPL-style), contact labels; the skeleton is tests/golden/kinopt/skeleton.bvh
   skeleton.npz    update_skeleton(...) of the reference: fitted offsets
-  funjac.npz      fun_anim_for_projection / jac_anim_for_projection_sparse of the reference at two points x (stage weights
-                  with and without the floor term)
+  funjac.npz      fun_anim_for_projection of the reference at two points x_a, x_b (stage weights without and with the
+                  floor term), with the weights and floor plane it was evaluated with
+  jac_a.npz,      jac_anim_for_projection_sparse of the reference at x_a resp. x_b, stored as CSR matrices
+  jac_b.npz       (scipy.sparse.save_npz: about 1 % of the entries are non-zero)
   run.npz         the reference's full optimize_trajectory(...) output on the clip: final x is not exposed by the
                   reference, so: final joint positions, re-projected 2D points, floor normal / point, refined contact labels,
                   and the objective 0.5 |f|^2 of the returned animation under the final-stage weights
@@ -15,6 +17,7 @@ import os
 import sys
 
 import numpy as np
+import scipy.sparse as sp
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, HERE)
@@ -118,7 +121,9 @@ def main():
         args = (sk, poses3D, root_pos, j2n, normal, point, pw, dw, np.arange(J), np.arange(J), ot.SMOOTH_WEIGHTS, vel, 1000.0, 0.1, 0.5, 0.3, 10.0, fw)
         fj["x_" + tag] = x
         fj["f_" + tag] = ot.fun_anim_for_projection(x, *args)
-        fj["J_" + tag] = np.asarray(ot.jac_anim_for_projection_sparse(x, *args).todense())
+        jac = sp.csr_matrix(ot.jac_anim_for_projection_sparse(x, *args))
+        jac.eliminate_zeros()
+        sp.save_npz(os.path.join(OUT, "jac_%s.npz" % tag), jac)
     np.savez_compressed(os.path.join(OUT, "funjac.npz"), normal=normal, point=point, pw=pw, dw=dw, j2n=j2n, **fj)
 
     # the full run

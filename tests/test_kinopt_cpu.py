@@ -36,6 +36,7 @@ def test_skeleton_fit_and_weights_match_reference(chd, data):
 
 @pytest.mark.parametrize("tag,floor_w", [("a", 0.0), ("b", 10.0)])
 def test_residual_and_jacobian_vs_reference(chd, data, tag, floor_w):
+    import scipy.sparse
     import torch
     ko = chd.kinopt
     fj, F = data["fj"], data["F"]
@@ -46,7 +47,7 @@ def test_residual_and_jacobian_vs_reference(chd, data, tag, floor_w):
     assert f.shape == fj["f_" + tag].shape
     # the reference's quaternion path carries 1e-10 relative noise (axis / (|axis| + 1e-10)); projection weight 1000
     np.testing.assert_allclose(f, fj["f_" + tag], rtol=0, atol=2e-7)
-    Jm, Jr = m.dense_jacobian(x, w).numpy(), fj["J_" + tag]
+    Jm, Jr = m.dense_jacobian(x, w).numpy(), scipy.sparse.load_npz(os.path.join(G, "jac_%s.npz" % tag)).toarray()
     assert Jm.shape == Jr.shape
     nproj = F * 28 * 2
     np.testing.assert_allclose(Jm[nproj:], Jr[nproj:], rtol=0, atol=1e-6)          # every group but the projection term
